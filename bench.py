@@ -80,6 +80,8 @@ def parse_args():
     p.add_argument("--cpu-sample-seconds", type=float, default=12.0)
     p.add_argument("--no-cpu-baseline", action="store_true")
     p.add_argument("--no-next-rows", action="store_true")
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="write what the last timed step returned (keys, distances, counts, both counters) as DIR/<name>.npy")
     p.add_argument("--builder", default="gpu", choices=["gpu", "reference"],
                    help="who builds the graph both arms search: the GPU builder (default) or the reference on the host cores")
     p.add_argument("--parallelism", default=None, choices=["replica", "shard"],
@@ -448,6 +450,26 @@ def measure_next_rows(a, index, ref, batch: np.ndarray, k: int, threads: int) ->
     return out
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, keys, distances, counts, computed, visited) -> None:
+    """The arrays search_device returned for one batch, as float64 (keys, counts, counters: exact below 2**53) and float32
+    (distances, bit for bit; padding stays NaN). A 4096-query batch at k = 10 is about 0.6 MB. A batch larger than
+    DUMP_LIMIT_BYTES in all is cut to a fixed, seeded sample of its rows, whose numbers go to rows.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    b, k = keys.shape
+    per_row = k * (8 + 4) + 3 * 8
+    rows = None
+    if b * per_row > DUMP_LIMIT_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(b, (DUMP_LIMIT_BYTES - 4096) // (per_row + 8), replace=False))
+        np.save(os.path.join(out_dir, "rows.npy"), rows.astype(np.float64))
+    for name, t, dtype in (("keys", keys, np.float64), ("distances", distances, np.float32), ("counts", counts, np.float64),
+                           ("computed_distances", computed, np.float64), ("visited_members", visited, np.float64)):
+        a = t.cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), (a if rows is None else a[rows]).astype(dtype))
+
+
 def run_b200_arm(a):
     import torch
     import torch.distributed as dist
@@ -549,6 +571,8 @@ def run_b200_arm(a):
     barrier()
     if ncu_range:
         torch.cuda.profiler.stop()
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, keys_dev, dist_dev, cnt_dev, comp_dev, vis_dev)
     launches = index.kernel_launches - launches0
     elapsed_ms = ev0.elapsed_time(ev1)
     t = torch.tensor([elapsed_ms], device=device)
@@ -602,8 +626,10 @@ def run_b200_arm(a):
     # ---- CPU baseline on a bounded sample + full-size parity (rank 0, N=1 only) ----
     cpu = None
     next_rows = None
-    if world == 1 and not a.no_cpu_baseline:
-        from oracle import bindings
+    from oracle import bindings
+    if world == 1 and not a.no_cpu_baseline and bindings.ref_lib("perf") is None:
+        log("cpu_baseline skipped: the reference library (oracle/_ref) is not built")
+    elif world == 1 and not a.no_cpu_baseline:
         threads_all = host_threads()
         t0 = time.time()
         if blob is None:

@@ -5,7 +5,7 @@ package ``usearch_b200`` never does.
 
 * :class:`RefIndex`  — the unmodified reference (oracle/_ref/libusearch_ref_*.so, built from
   /root/reference by oracle/build.py).
-* :class:`PortIndex` — the plain-C restatement (oracle/liboracle.so).
+* :class:`PortIndex`, :func:`port_exact_search` — the plain-C restatement (oracle/liboracle.so).
 """
 from __future__ import annotations
 
@@ -274,6 +274,11 @@ def port_lib() -> C.CDLL:
     lib.oracle_distance.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
     lib.oracle_search_many.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int,
                                        _u64p, _f32p, _u64p, _u64p, _u64p]
+    lib.oracle_filtered_search_many.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int,
+                                                _u64p, C.c_size_t, _u64p, _f32p, _u64p, _u64p, _u64p]
+    lib.oracle_exact_search.restype = C.c_int
+    lib.oracle_exact_search.argtypes = [C.c_void_p, C.c_size_t, C.c_size_t, C.c_void_p, C.c_size_t, C.c_size_t, C.c_int,
+                                        C.c_int, C.c_size_t, C.c_size_t, _u64p, _f32p]
     lib.oracle_cluster_many.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_size_t, C.c_size_t, _u64p, _f32p, _u64p, _u64p]
     lib.oracle_cast_from_f32.restype = C.c_size_t
     lib.oracle_cast_from_f32.argtypes = [C.c_int, _f32p, C.c_size_t, C.c_void_p]
@@ -324,6 +329,19 @@ class PortIndex:
                                     _ptr(computed, _u64p), _ptr(visited, _u64p))
         return keys, dist, counts, computed, visited
 
+    def filtered_search(self, queries: np.ndarray, k: int, allowed_keys: np.ndarray, threads: int = 1):
+        """filtered_search with the predicate "key in allowed_keys"."""
+        queries = np.ascontiguousarray(queries)
+        allowed = np.sort(np.ascontiguousarray(allowed_keys, dtype=np.uint64))
+        nq = queries.shape[0]
+        keys = np.zeros((nq, k), dtype=np.uint64)
+        dist = np.zeros((nq, k), dtype=np.float32)
+        counts, computed, visited = (np.zeros(nq, dtype=np.uint64) for _ in range(3))
+        self.lib.oracle_filtered_search_many(self.h, _ptr(queries), nq, queries.strides[0] if nq else 0, k, threads, 0,
+                                             _ptr(allowed, _u64p), allowed.size, _ptr(keys, _u64p), _ptr(dist, _f32p),
+                                             _ptr(counts, _u64p), _ptr(computed, _u64p), _ptr(visited, _u64p))
+        return keys, dist, counts, computed, visited
+
     def cluster(self, queries: np.ndarray, level: int):
         queries = np.ascontiguousarray(queries)
         nq = queries.shape[0]
@@ -334,3 +352,18 @@ class PortIndex:
         self.lib.oracle_cluster_many(self.h, _ptr(queries), nq, queries.strides[0] if nq else 0, level, _ptr(keys, _u64p),
                                      _ptr(dist, _f32p), _ptr(computed, _u64p), _ptr(visited, _u64p))
         return keys, dist, computed, visited
+
+
+def port_exact_search(dataset: np.ndarray, queries: np.ndarray, k: int, *, metric: str, scalar: str, dims: int):
+    """The plain-C restatement of exact_search_t over raw matrices (pinned metrics); keys are dataset row numbers."""
+    lib = port_lib()
+    dataset = np.ascontiguousarray(dataset)
+    queries = np.ascontiguousarray(queries)
+    nq = queries.shape[0]
+    keys = np.zeros((nq, k), dtype=np.uint64)
+    dist = np.zeros((nq, k), dtype=np.float32)
+    rc = lib.oracle_exact_search(_ptr(dataset), dataset.shape[0], dataset.strides[0], _ptr(queries), nq, queries.strides[0],
+                                 METRIC[metric], SCALAR[scalar], dims, k, _ptr(keys, _u64p), _ptr(dist, _f32p))
+    if rc:
+        raise RuntimeError(f"oracle_exact_search failed: {rc}")
+    return keys, dist

@@ -302,6 +302,23 @@ static float measure(oracle_index_t const* ix, context_t* c, void const* q, uint
 
 /* ---------- the search path --------------------------------------------------------------- */
 
+/* The predicate of index_dense_gt (index_dense.hpp:2071-2077): not a removed member and, for filtered_search, a key
+ * in the caller's set (sorted ascending; NULL admits every key). */
+typedef struct { uint64_t const* keys; size_t count; } allowed_t;
+
+static int admits(oracle_index_t const* ix, allowed_t const* allowed, uint32_t slot) {
+    uint64_t key = node_key(ix, slot);
+    if (key == ix->free_key) return 0;
+    if (!allowed || !allowed->keys) return 1;
+    size_t lo = 0, hi = allowed->count;
+    while (lo < hi) {
+        size_t mid = lo + (hi - lo) / 2;
+        if (allowed->keys[mid] < key) lo = mid + 1;
+        else hi = mid;
+    }
+    return lo < allowed->count && allowed->keys[lo] == key;
+}
+
 /* search_for_one_ (index.hpp:3963-4003): greedy descent from begin_level down to level 1 */
 static uint32_t search_for_one(oracle_index_t const* ix, context_t* c, void const* q, uint32_t closest,
                                int64_t begin_level, int64_t end_level) {
@@ -325,7 +342,8 @@ static uint32_t search_for_one(oracle_index_t const* ix, context_t* c, void cons
 }
 
 /* search_to_find_in_base_ (index.hpp:4175-4246): best-first expansion over layer 0 */
-static int search_to_find_in_base(oracle_index_t const* ix, context_t* c, void const* q, uint32_t start, size_t expansion) {
+static int search_to_find_in_base(oracle_index_t const* ix, context_t* c, void const* q, uint32_t start, size_t expansion,
+                                  allowed_t const* allowed) {
     heap_t* next = &c->next;
     sorted_t* top = &c->top;
     visits_t* visits = &c->visits;
@@ -339,7 +357,7 @@ static int search_to_find_in_base(oracle_index_t const* ix, context_t* c, void c
     candidate_t seed = {-radius, start};
     next->e[next->size++] = seed; /* insert_reserved into an empty heap */
     visits_set(visits, start);
-    if (node_key(ix, start) != ix->free_key) { /* predicate: index_dense.hpp:2071-2077 */
+    if (admits(ix, allowed, start)) {
         candidate_t t = {radius, start};
         sorted_insert_reserved(top, t);
     }
@@ -360,7 +378,7 @@ static int search_to_find_in_base(oracle_index_t const* ix, context_t* c, void c
             if (top->size < top_limit || d < radius) {
                 candidate_t neg = {-d, succ};
                 if (!heap_insert(next, neg)) return 0;
-                if (node_key(ix, succ) != ix->free_key) {
+                if (admits(ix, allowed, succ)) {
                     candidate_t pos = {d, succ};
                     sorted_insert(top, pos, top_limit);
                     radius = top->e[top->size - 1].distance;
@@ -372,10 +390,10 @@ static int search_to_find_in_base(oracle_index_t const* ix, context_t* c, void c
 }
 
 /* search_exact_ (index.hpp:4251-4268) */
-static void search_exact(oracle_index_t const* ix, context_t* c, void const* q, size_t count) {
+static void search_exact(oracle_index_t const* ix, context_t* c, void const* q, size_t count, allowed_t const* allowed) {
     c->top.size = 0;
     for (uint64_t i = 0; i < ix->size; ++i) {
-        if (node_key(ix, (uint32_t)i) == ix->free_key) continue;
+        if (!admits(ix, allowed, (uint32_t)i)) continue;
         candidate_t t = {measure(ix, c, q, (uint32_t)i), (uint32_t)i};
         sorted_insert(&c->top, t, count);
     }
@@ -387,7 +405,8 @@ static uint32_t const SNAN_BITS = 0x7FA00000u; /* std::numeric_limits<float>::si
  * The query is already in the index's scalar kind. Returns the number of results found;
  * always writes `wanted` output slots. */
 static size_t search_one(oracle_index_t const* ix, context_t* c, void const* q, size_t wanted, size_t expansion_cfg,
-                         int exact, uint64_t* keys, float* distances, uint64_t* computed, uint64_t* visited) {
+                         int exact, allowed_t const* allowed, uint64_t* keys, float* distances, uint64_t* computed,
+                         uint64_t* visited) {
     size_t count = 0;
     uint64_t computed0 = c->computed_distances, cycles0 = c->iteration_cycles;
     c->top.size = 0;
@@ -396,7 +415,7 @@ static size_t search_one(oracle_index_t const* ix, context_t* c, void const* q, 
         if (exact) {
             size_t cap = wanted + 1;
             if (c->top.capacity < cap) { c->top.e = (candidate_t*)realloc(c->top.e, cap * sizeof(candidate_t)); c->top.capacity = cap; }
-            search_exact(ix, c, q, wanted);
+            search_exact(ix, c, q, wanted, allowed);
         } else {
             size_t expansion = expansion_cfg > wanted ? expansion_cfg : wanted;
             heap_reserve(&c->next, expansion);
@@ -405,7 +424,7 @@ static size_t search_one(oracle_index_t const* ix, context_t* c, void const* q, 
                 c->top.capacity = expansion + 1;
             }
             uint32_t closest = search_for_one(ix, c, q, (uint32_t)ix->entry_slot, (int64_t)ix->max_level, 0);
-            search_to_find_in_base(ix, c, q, closest, expansion);
+            search_to_find_in_base(ix, c, q, closest, expansion, allowed);
         }
         if (c->top.size > wanted) c->top.size = wanted; /* shrink */
         count = c->top.size;
@@ -429,6 +448,7 @@ typedef struct {
     uint8_t const* queries;
     size_t nq, stride, wanted, expansion;
     int exact;
+    allowed_t allowed;
     uint64_t *keys, *counts, *computed, *visited;
     float* distances;
     size_t begin, end;
@@ -439,17 +459,18 @@ static void* worker(void* arg) {
     context_t c;
     memset(&c, 0, sizeof(c));
     for (size_t i = j->begin; i < j->end; ++i)
-        j->counts[i] = search_one(j->ix, &c, j->queries + i * j->stride, j->wanted, j->expansion, j->exact,
+        j->counts[i] = search_one(j->ix, &c, j->queries + i * j->stride, j->wanted, j->expansion, j->exact, &j->allowed,
                                   j->keys + i * j->wanted, j->distances + i * j->wanted,
                                   j->computed ? j->computed + i : NULL, j->visited ? j->visited + i : NULL);
     context_free(&c);
     return NULL;
 }
 
-/* Batch driver: contiguous chunks per thread, like executor_stl_t::dynamic (index_plugins.hpp:668-690). */
-void oracle_search_many(oracle_index_t const* ix, void const* queries, size_t nq, size_t stride_bytes, size_t wanted,
-                        size_t threads, int exact, uint64_t* keys, float* distances, uint64_t* counts,
-                        uint64_t* computed, uint64_t* visited) {
+/* Batch driver: contiguous chunks per thread, like executor_stl_t::dynamic (index_plugins.hpp:668-690).
+ * `allowed_keys` (sorted ascending) makes it filtered_search (index_dense.hpp:774-779); NULL searches every member. */
+void oracle_filtered_search_many(oracle_index_t const* ix, void const* queries, size_t nq, size_t stride_bytes,
+                                 size_t wanted, size_t threads, int exact, uint64_t const* allowed_keys, size_t allowed_count,
+                                 uint64_t* keys, float* distances, uint64_t* counts, uint64_t* computed, uint64_t* visited) {
     if (threads < 1) threads = 1;
     if (threads > nq) threads = nq ? nq : 1;
     job_t* jobs = (job_t*)calloc(threads, sizeof(job_t));
@@ -457,7 +478,7 @@ void oracle_search_many(oracle_index_t const* ix, void const* queries, size_t nq
     size_t per = (nq + threads - 1) / threads;
     for (size_t t = 0; t < threads; ++t) {
         job_t j = {ix, (uint8_t const*)queries, nq, stride_bytes, wanted, ix->expansion_search, exact,
-                   keys, counts, computed, visited, distances, t * per, (t + 1) * per < nq ? (t + 1) * per : nq};
+                   {allowed_keys, allowed_count}, keys, counts, computed, visited, distances, t * per, (t + 1) * per < nq ? (t + 1) * per : nq};
         if (j.begin > nq) j.begin = nq;
         jobs[t] = j;
         if (threads == 1) worker(&jobs[t]);
@@ -467,6 +488,36 @@ void oracle_search_many(oracle_index_t const* ix, void const* queries, size_t nq
         for (size_t t = 0; t < threads; ++t) pthread_join(tids[t], NULL);
     free(jobs);
     free(tids);
+}
+
+void oracle_search_many(oracle_index_t const* ix, void const* queries, size_t nq, size_t stride_bytes, size_t wanted,
+                        size_t threads, int exact, uint64_t* keys, float* distances, uint64_t* counts,
+                        uint64_t* computed, uint64_t* visited) {
+    oracle_filtered_search_many(ix, queries, nq, stride_bytes, wanted, threads, exact, NULL, 0, keys, distances, counts,
+                                computed, visited);
+}
+
+/* exact_search_t (index_plugins.hpp:2071-2164) over raw matrices: metric(dataset row, query) for every pair, the `wanted`
+ * smallest distances of each query in ascending order, keys = dataset row numbers (the order among equal distances is
+ * unspecified there: std::partial_sort). Returns 0, or -1 for an unknown metric / scalar pair or wanted > n. */
+int oracle_exact_search(void const* dataset, size_t n, size_t dataset_stride, void const* queries, size_t nq,
+                        size_t queries_stride, int metric_kind, int scalar_kind, size_t dimensions, size_t wanted,
+                        uint64_t* keys, float* distances) {
+    oracle_metric_t metric = pick_metric((uint8_t)metric_kind, (uint8_t)scalar_kind);
+    size_t third = scalar_kind == SK_B1 ? (dimensions + 7) / 8 : dimensions;
+    if (!metric || wanted > n) return -1;
+    sorted_t top = {(candidate_t*)malloc((wanted + 1) * sizeof(candidate_t)), 0, wanted + 1};
+    for (size_t q = 0; q < nq; ++q) {
+        void const* query = (uint8_t const*)queries + q * queries_stride;
+        top.size = 0;
+        for (size_t i = 0; i < n; ++i) {
+            candidate_t c = {metric((uint8_t const*)dataset + i * dataset_stride, query, third), (uint32_t)i};
+            sorted_insert(&top, c, wanted);
+        }
+        for (size_t i = 0; i < wanted; ++i) keys[q * wanted + i] = top.e[i].slot, distances[q * wanted + i] = top.e[i].distance;
+    }
+    free(top.e);
+    return 0;
 }
 
 /* Query-side casts from f32 (index_plugins.hpp:1105-1224): used to validate the device casts.

@@ -1,9 +1,11 @@
 """GPU-assisted add (SURVEY.md §8f N4; csrc/builder.cu) and the by-key half of the C ABI, on one GPU.
 
 A GPU-built graph is not bit-identical to a reference-built one (neither are two multi-threaded reference builds), so the
-bar is DESIGN.md §9: structure invariants, and the REFERENCE search on the GPU-built file reaching the recall and the work
-per query it reaches on the reference-built file. Our own search on our own graph must still equal the reference's
-search on that same graph bit for bit."""
+bar is DESIGN.md §9: structure invariants, and the reference search (the pinned plain-C oracle) on the GPU-built file
+reaching the recall and the work per query the reference reached on its own file of the same collection
+(tests/golden/build_quality.json). Our own search on our own graph must still equal the oracle's search on that same
+graph bit for bit."""
+import json
 import os
 import sys
 import threading
@@ -32,7 +34,6 @@ def test_gpu_built_graph_is_as_good_as_a_reference_built_one(metric, scalar, n, 
     from usearch_b200.index import Index
     base, queries = common.make_collection(n, d, scalar, 400)
     keys = np.arange(n, dtype=np.uint64)
-    ref, ref_blob = common.build_reference_blob(base, metric, scalar, d, m, threads=16)
     index = Index(ndim=d, metric=metric, dtype=scalar, connectivity=m, expansion_add=128)
     index.add(keys, base)
     assert len(index) == n
@@ -40,20 +41,13 @@ def test_gpu_built_graph_is_as_good_as_a_reference_built_one(metric, scalar, n, 
     rep = structure_report(gpu_blob)
     assert rep["n_problems"] == 0, rep["problems"]
     truth = hamming_truth(base, queries, 10) if scalar == "b1" else exact_truth(base, queries, metric, 10)
-    searcher = bindings.RefIndex("parity")
-    got = {}
-    for label, blob in (("ref", ref_blob), ("gpu", gpu_blob)):
-        searcher.load(blob)
-        searcher.change_expansion_search(64)
-        k, _, _, comp, _ = searcher.search(queries, 10, threads=16)
-        got[label] = (recall(k, truth), float(comp.mean()))
+    with open(os.path.join(common.GOLDEN, "build_quality.json")) as f:
+        ref = json.load(f)[f"{metric}/{scalar}/{n}/{d}/{m}"]  # the reference's search of its own graph, ef = 64
+    want = bindings.PortIndex(gpu_blob, 64).search(queries, 10, threads=16)
+    got = {"ref": (ref["recall"], ref["computed_per_query"]), "gpu": (recall(want[0], truth), float(want[3].mean()))}
     assert got["gpu"][0] >= got["ref"][0] - 0.01, got
     assert abs(got["gpu"][1] - got["ref"][1]) <= 0.08 * got["ref"][1], got
-    # same graph => our search and the reference's agree bit for bit
-    searcher.load(gpu_blob)
-    searcher.pin_metric(True)
-    searcher.change_expansion_search(64)
-    want = searcher.search(queries, 10, threads=16)
+    # same graph => our search and the oracle's agree bit for bit
     index.expansion_search = 64
     mine = index.search(queries, 10, stats=True)
     common.assert_same_results(want, (mine.keys, mine.distances, mine.counts, index.last_computed, index.last_visited), "gpu graph")
@@ -86,11 +80,12 @@ def test_incremental_adds_grow_the_index_and_find_themselves():
 
 
 def test_lookups_and_edits_by_key():
+    from usearch_b200 import v2format
     from usearch_b200.index import Index, load_library
     import ctypes as C
     n, d = 3000, 48
     base, queries = common.make_collection(n, d, "f32", 64)
-    ref, blob = common.build_reference_blob(base, "ip", "f32", d, 16, threads=8, keys=np.arange(n, dtype=np.uint64) * 3)
+    blob = common.build_graph_blob(base, "ip", "f32", d, 16, keys=np.arange(n, dtype=np.uint64) * 3)
     index = Index.restore(blob)                             # lookups work on a loaded file too
     assert index.contains(30) and not index.contains(31) and index.count(30) == 1 and index.count(31) == 0
     assert np.array_equal(index.get(30), base[10]) and index.get(31) is None
@@ -110,10 +105,11 @@ def test_lookups_and_edits_by_key():
     assert len(index) == n - 1 and not index.contains(victim)
     after = index.search(queries, 10)
     assert victim not in after.keys.tolist()[0]
-    ref.remove(victim)                                      # the reference after the same removal: same answers
-    ref.pin_metric(True)
-    ref.change_expansion_search(64)
-    want = ref.search(queries, 10, threads=8)
+    # the file after the same removal, modelled as the reference's remove does it (the key becomes the free key, the
+    # links stay; golden fixture ip_f32_n1500_d48_removed): same answers
+    graph = v2format.loads(blob)
+    graph.keys[graph.keys == victim] = v2format.FREE_KEY
+    want = bindings.PortIndex(v2format.dumps(graph), 64).search(queries, 10, threads=8)
     assert np.array_equal(after.keys, want[0]) and np.array_equal(after.distances.view(np.uint32), want[1].view(np.uint32))
     # rename
     other = int(before.keys[1, 0])
@@ -129,7 +125,7 @@ def test_concurrent_single_query_callers_are_gathered():
     from usearch_b200.index import Index
     n, d = 4000, 64
     base, queries = common.make_collection(n, d, "f32", 256)
-    ref, blob = common.build_reference_blob(base, "cos", "f32", d, 16, threads=8)
+    blob = common.build_graph_blob(base, "cos", "f32", d, 16)
     index = Index.restore(blob)
     index.expansion_search = 64
     want = index.search(queries, 10)
@@ -148,7 +144,7 @@ def test_concurrent_single_query_callers_are_gathered():
 
 
 def _cpu_indexes_merge(per_shard, k):
-    """`Indexes`-style merge of per-shard reference results (python/lib.cpp:350-391) with the deterministic order."""
+    """`Indexes`-style merge of per-shard CPU results (python/lib.cpp:350-391) with the deterministic order."""
     nq = per_shard[0][0].shape[0]
     out_k = np.zeros((nq, k), np.uint64)
     out_d = np.full((nq, k), np.array(0x7FA00000, dtype=np.uint32).view(np.float32), np.float32)
@@ -167,18 +163,17 @@ def _cpu_indexes_merge(per_shard, k):
 
 @pytest.mark.parametrize("metric,scalar,d,m,G", [("cos", "f32", 96, 16, 3), ("hamming", "b1", 128, 16, 4), ("ip", "i8", 128, 16, 2)])
 def test_sharded_search_matches_the_cpu_indexes_merge(metric, scalar, d, m, G):
-    """SURVEY §8e parity target: the CPU `Indexes` search over the SAME G serialised shards, merged by (distance, shard,
-    position). Each shard is searched on the GPU; the merge kernel does the exchange step's second half."""
+    """SURVEY §8e parity target: the CPU `Indexes` search (the pinned oracle per shard) over the SAME G serialised shards,
+    merged by (distance, shard, position). Each shard is searched on the GPU; the merge kernel does the exchange step's
+    second half."""
     from usearch_b200.index import Index, merge_topk
     n, k, ef = 9000, 10, 64
     base, queries = common.make_collection(n, d, scalar, 200)
     keys = np.arange(n, dtype=np.uint64)
     cpu, gpu = [], []
     for r in range(G):
-        ref, blob = common.build_reference_blob(base[r::G], metric, scalar, d, m, threads=16, keys=keys[r::G])
-        ref.pin_metric(True)
-        ref.change_expansion_search(ef)
-        want = ref.search(queries, k, threads=16)
+        blob = common.build_graph_blob(base[r::G], metric, scalar, d, m, keys=keys[r::G])
+        want = bindings.PortIndex(blob, ef).search(queries, k, threads=16)
         cpu.append((want[0], want[1], want[2]))
         index = Index.restore(blob)
         index.expansion_search = ef
@@ -212,16 +207,20 @@ def test_merge_kernel_equals_its_torch_specification():
     assert np.array_equal(got.distances.view(np.uint32), wd.numpy().view(np.uint32))
 
 
-def test_enqueue_then_finish_equals_the_blocking_calls():
+def test_enqueue_then_finish_equals_the_blocking_calls(tmp_path):
     """usearch_b200_search_many_enqueue x3 + one _finish == three usearch_b200_search_many_device calls, with scratch small
-    enough (test hook) that some queries overflow and have to be retried by _finish."""
+    enough (test hook) that some queries overflow and have to be retried by _finish. The graph is built here, outside
+    the process whose search runs under the test hooks."""
     import subprocess
+    base, _ = common.make_collection(6000, 64, "f32", 1)
+    path = str(tmp_path / "graph.usearch")
+    common.build_graph_blob(base, "cos", "f32", 64, 16).tofile(path)
     code = (
         "import sys; sys.path.insert(0, %r); sys.path.insert(0, %r)\n"
         "import numpy as np, torch, common\n"
         "from usearch_b200.index import Index\n"
         "base, q = common.make_collection(6000, 64, 'f32', 384)\n"
-        "ref, blob = common.build_reference_blob(base, 'cos', 'f32', 64, 16, threads=8)\n"
+        "blob = np.fromfile(%r, dtype=np.uint8)\n"
         "index = Index.restore(blob); index.expansion_search = 64\n"
         "dev = torch.device('cuda', 0)\n"
         "qd = torch.from_numpy(q).to(dev)\n"
@@ -236,29 +235,31 @@ def test_enqueue_then_finish_equals_the_blocking_calls():
         "want = index.search(q, 10)\n"
         "assert np.array_equal(torch.cat([s[0] for s in deferred]).cpu().numpy().astype(np.uint64), want.keys)\n"
         "print('ENQUEUE_OK')\n"
-    ) % (common.ROOT, os.path.join(common.ROOT, "tests"))
+    ) % (common.ROOT, os.path.join(common.ROOT, "tests"), path)
     env = dict(os.environ, USEARCH_B200_VISITED="hash", USEARCH_B200_SCRATCH_SHRINK="64")
     out = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=600)
     assert out.returncode == 0 and "ENQUEUE_OK" in out.stdout, out.stdout[-2000:] + out.stderr[-2000:]
 
 
 def test_adding_to_a_loaded_reference_built_index():
-    """`load` a file written by the reference, then keep adding on the GPU (capacity grows from the file's size), save, and
-    let the reference search the result: every member, old and new, is its own nearest neighbour."""
+    """`load` a file written by the reference (a committed golden fixture), then keep adding on the GPU (capacity grows
+    from the file's size), save, and let the reference search (the pinned oracle) search the result: every member, old
+    and new, is its own nearest neighbour."""
+    from usearch_b200 import v2format
     from usearch_b200.index import Index
-    n0, n1, d = 4000, 3000, 64
-    base, _ = common.make_collection(n0 + n1, d, "f32", 1)
-    ref, blob = common.build_reference_blob(base[:n0], "cos", "f32", d, 16, threads=8)
+    blob = np.load(os.path.join(common.GOLDEN, "cos_f32_n2000_d64.npz"))["blob"]
+    graph = v2format.loads(blob)
+    n0, n1, d = graph.size, 3000, graph.dimensions
+    assert graph.metric == "cos" and graph.scalar == "f32" and np.array_equal(graph.keys, np.arange(n0, dtype=np.uint64))
+    added, _ = common.make_collection(n1, d, "f32", 1, seed=7)
+    base = np.concatenate([graph.vectors.view(np.float32).reshape(n0, d), added])
     index = Index.restore(blob)
     assert len(index) == n0
     index.add(np.arange(n0, n0 + n1, dtype=np.uint64), base[n0:])
     assert len(index) == n0 + n1
     rep = structure_report(index.save())
     assert rep["n_problems"] == 0, rep["problems"]
-    searcher = bindings.RefIndex("parity")
-    searcher.load(index.save())
-    searcher.change_expansion_search(64)
-    keys, dist, _, _, _ = searcher.search(base, 1, threads=16)
+    keys, dist, _, _, _ = bindings.PortIndex(index.save(), 64).search(base, 1, threads=16)
     assert (keys[:, 0] == np.arange(n0 + n1, dtype=np.uint64)).mean() > 0.995
     # clear -> the handle is reusable for a new collection
     index.clear()

@@ -1,6 +1,7 @@
 """GPU parity of the brute-force path (SURVEY.md §8 N1): `search(exact=True)` on a frozen index against
 index_gt::search_exact_ (index.hpp:4251-4268), and `usearch_exact_search` against exact_search_t
-(index_plugins.hpp:2071-2164), both run by the unmodified reference on the same inputs."""
+(index_plugins.hpp:2071-2164), both as the pinned plain-C oracle restates them (pinned to the reference's own outputs
+by tests/golden). Graphs come from this project's builder, removed members from its `remove` (common.build_graph_blob)."""
 import numpy as np
 import pytest
 
@@ -37,12 +38,8 @@ def test_index_exact_search_matches_reference(metric, scalar, n, d, k, nq, remov
     base, q = common.make_collection(n, d, scalar, nq)
     base[n // 2:n // 2 + 40] = base[:40]          # duplicated vectors under different keys: equal distances
     keys = np.arange(n, dtype=np.uint64) * 7 + 3
-    ref, _ = common.build_reference_blob(base, metric, scalar, d, 8, expansion_add=16, threads=16, keys=keys)
-    for key in keys[5:5 + removed]:
-        ref.remove(int(key))
-    blob = ref.save()
-    ref.pin_metric(True)
-    want = ref.search(q, k, threads=8, exact=True)
+    blob = common.build_graph_blob(base, metric, scalar, d, 8, expansion_add=16, keys=keys, removed=keys[5:5 + removed])
+    want = bindings.PortIndex(blob).search(q, k, threads=8, exact=True)
     index = Index.restore(blob)
     got = index.search(q, k, exact=True)
     common.assert_same_results(want[:3], (got.keys, got.distances, got.counts), f"exact gpu vs reference [{metric}/{scalar}]")
@@ -53,9 +50,8 @@ def test_index_exact_search_matches_reference(metric, scalar, n, d, k, nq, remov
 def test_index_exact_search_with_fewer_members_than_wanted():
     from usearch_b200.index import Index
     base, q = common.make_collection(7, 32, "f32", 5)
-    ref, blob = common.build_reference_blob(base, "l2sq", "f32", 32, 8, threads=1)
-    ref.pin_metric(True)
-    want = ref.search(q, 10, threads=1, exact=True)
+    blob = common.build_graph_blob(base, "l2sq", "f32", 32, 8)
+    want = bindings.PortIndex(blob).search(q, 10, threads=1, exact=True)
     got = Index.restore(blob).search(q, 10, exact=True)
     assert (got.counts == 7).all()
     common.assert_same_results(want[:3], (got.keys, got.distances, got.counts), "exact, k > n")
@@ -66,7 +62,7 @@ def test_index_exact_search_agrees_with_graph_search_at_full_expansion():
     with ef = n the graph search finds (nearly) everything the scan does."""
     from usearch_b200.index import Index
     base, q = common.make_collection(2000, 64, "f32", 64, iid=True)
-    _, blob = common.build_reference_blob(base, "l2sq", "f32", 64, 16, threads=1)
+    blob = common.build_graph_blob(base, "l2sq", "f32", 64, 16)
     index = Index.restore(blob)
     exact = index.search(q, 10, exact=True)
     index.expansion_search = 2000
@@ -97,10 +93,8 @@ FREE_CASES = [
 @pytest.mark.parametrize("metric,scalar,n,d,k,nq", FREE_CASES)
 def test_free_exact_search_matches_reference(metric, scalar, n, d, k, nq):
     from usearch_b200.index import exact_search
-    if not common.have_reference():
-        pytest.skip("reference library not built")
     base, q = common.make_collection(n, d, scalar, nq)
-    wk, wd = bindings.ref_exact_search(base, q, k + 1, metric=metric, scalar=scalar, dims=d, pinned=True)
+    wk, wd = bindings.port_exact_search(base, q, k + 1, metric=metric, scalar=scalar, dims=d)
     got = exact_search(base, q, k, metric=metric, dtype=scalar)
     assert np.array_equal(got.distances.view(np.uint32), wd[:, :k].view(np.uint32)), "distance bits differ"
     # labels are defined wherever the distance is unique in the row (std::partial_sort leaves ties unspecified)
@@ -111,7 +105,7 @@ def test_free_exact_search_matches_reference(metric, scalar, n, d, k, nq):
     # and every reported label really has the reported distance
     for row in range(0, nq, 7):
         members = base[got.keys[row].astype(np.int64)]
-        again = bindings.ref_exact_search(members, q[row:row + 1], k, metric=metric, scalar=scalar, dims=d, pinned=True)[1]
+        again = bindings.port_exact_search(members, q[row:row + 1], k, metric=metric, scalar=scalar, dims=d)[1]
         assert np.array_equal(again[0].view(np.uint32), got.distances[row].view(np.uint32))
 
 
@@ -132,8 +126,8 @@ def test_cluster_matches_reference(metric, scalar, n, d, m):
     """index_dense_gt::cluster(vector, level): the descent of the search kernel stopped at `level`."""
     from usearch_b200.index import Index
     base, q = common.make_collection(n, d, scalar, 300)
-    ref, blob = common.build_reference_blob(base, metric, scalar, d, m, threads=16)
-    ref.pin_metric(True)
+    blob = common.build_graph_blob(base, metric, scalar, d, m)
+    ref = bindings.PortIndex(blob)
     index = Index.restore(blob)
     assert index.max_level == ref.max_level >= 3
     for level in (0, 1, 2, ref.max_level, ref.max_level + 2):
@@ -167,13 +161,11 @@ def test_i8_exact_kernels_agree_with_the_reference(kernel):
         "    base, q = common.make_collection(n, d, 'i8', nq)\n"
         "    base[n // 2:n // 2 + 30] = base[:30]\n"
         "    keys = np.arange(n, dtype=np.uint64) * 5 + 1\n"
-        "    ref, _ = common.build_reference_blob(base, metric, 'i8', d, 8, expansion_add=16, threads=16, keys=keys)\n"
-        "    for key in keys[3:3 + removed]: ref.remove(int(key))\n"
-        "    blob = ref.save(); ref.pin_metric(True)\n"
-        "    want = ref.search(q, k, threads=8, exact=True)\n"
+        "    blob = common.build_graph_blob(base, metric, 'i8', d, 8, expansion_add=16, keys=keys, removed=keys[3:3 + removed])\n"
+        "    want = bindings.PortIndex(blob).search(q, k, threads=8, exact=True)\n"
         "    got = Index.restore(blob).search(q, k, exact=True)\n"
         "    common.assert_same_results(want[:3], (got.keys, got.distances, got.counts), metric)\n"
-        "    wk, wd = bindings.ref_exact_search(base, q, k, metric=metric, scalar='i8', dims=d)\n"
+        "    wk, wd = bindings.port_exact_search(base, q, k, metric=metric, scalar='i8', dims=d)\n"
         "    free = exact_search(base, q, k, metric=metric, dtype='i8')\n"
         "    assert np.array_equal(free.distances.view(np.uint32), wd.view(np.uint32)), metric\n"
         "print('I8_EXACT_OK')\n"

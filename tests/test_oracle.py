@@ -1,7 +1,7 @@
 """CPU tests that PIN the oracle: the plain-C restatement (oracle/hnsw_oracle.c) against
-  (a) the committed golden fixtures produced by the unmodified reference (tests/golden/make_golden.py),
+  (a) the committed golden fixtures produced by the unmodified reference (tests/golden/make_golden*.py),
   (b) the tiny known-answer vectors the reference's own test-suites hold,
-  (c) the live reference library when oracle/_ref is available."""
+  (c) the live reference library when oracle/_ref is available (the same configurations, smaller, are in (a))."""
 import glob
 import os
 
@@ -190,26 +190,57 @@ def test_port_next_rows_match_golden(path):
         assert np.array_equal(cc, nr[f"{name}/cluster_computed"][i]) and np.array_equal(cv, nr[f"{name}/cluster_visited"][i])
 
 
+@pytest.mark.parametrize("path", FIXTURES, ids=[os.path.basename(p)[:-4] for p in FIXTURES])
+def test_port_filtered_and_free_exact_search_match_golden(path):
+    """filtered_search and exact_search_t over raw matrices of the plain-C port against what the reference returned on the
+    fixture graphs (tests/golden/port_extras.npz, made by make_golden_port_extras.py)."""
+    name = os.path.basename(path)[:-4]
+    g, px = np.load(path), np.load(os.path.join(common.GOLDEN, "port_extras.npz"))
+    graph = v2format.loads(g["blob"])
+    q, k = g["queries"], int(g["k"])
+    vectors = graph.vectors.view(bindings.SCALAR_NP[graph.scalar]).reshape(graph.size, -1)
+    fk, fd = bindings.port_exact_search(vectors, q, k + 1, metric=graph.metric, scalar=graph.scalar, dims=graph.dimensions)
+    wk, wd = px[f"{name}/free_keys"], px[f"{name}/free_distances"]
+    assert np.array_equal(fd.view(np.uint32), wd.view(np.uint32))
+    unique = wd[:, :k] != wd[:, 1:k + 1]  # std::partial_sort leaves the order of equal distances unspecified
+    unique[:, 1:] &= wd[:, 1:k] != wd[:, :k - 1]
+    assert np.array_equal(fk[:, :k][unique], wk[:, :k][unique])
+    if graph.scalar != "f32":
+        return
+    port = bindings.PortIndex(g["blob"], int(g["ef"]))
+    for i in range(3):
+        want = tuple(px[f"{name}/filtered_{i}_{f}"] for f in ("keys", "distances", "counts", "computed", "visited"))
+        got = port.filtered_search(q, k, px[f"{name}/filtered_{i}_allowed"], threads=2)
+        common.assert_same_results(want, got, f"{name} filtered {i}")
+
+
+def test_casts_match_golden():
+    """datagen.to_scalar (how the tests quantise f32 rows) and the port's casts equal the reference's cast_gt
+    (index_plugins.hpp:1105-1224) on the rows of tests/golden/port_extras.npz."""
+    import ctypes as C
+    px = np.load(os.path.join(common.GOLDEN, "port_extras.npz"))
+    x = px["cast/input"]
+    for scalar in ("f16", "bf16", "i8", "b1"):
+        want = px[f"cast/{scalar}"]
+        assert np.array_equal(common.datagen.to_scalar(x, scalar).view(np.uint8), want.view(np.uint8)), scalar
+        if scalar in ("i8", "b1"):
+            lib = bindings.port_lib()
+            for row, expect in zip(x, want):
+                out = np.zeros(bindings.bytes_per_vector(x.shape[1], scalar), dtype=np.uint8)
+                lib.oracle_cast_from_f32(bindings.SCALAR[scalar], row.ctypes.data_as(bindings._f32p), x.shape[1],
+                                         out.ctypes.data_as(C.c_void_p))
+                assert np.array_equal(out, expect.view(np.uint8)), scalar
+
+
 @pytest.mark.skipif(not common.have_reference(), reason="oracle/_ref not built")
 def test_port_matches_live_reference_on_random_small_cases():
     """Forty seeded random configurations at the small end (n from 1, k > n, ef < k, removed members, duplicate vectors,
     every scalar kind): graph search, exact search and cluster of the port against the reference, bit for bit."""
-    rng = np.random.default_rng(2026)
-    kinds = [("l2sq", "f32"), ("cos", "f32"), ("ip", "f32"), ("cos", "f16"), ("l2sq", "bf16"), ("ip", "i8"), ("cos", "i8"),
-             ("hamming", "b1"), ("tanimoto", "b1"), ("sorensen", "b1")]
-    for case in range(40):
-        metric, scalar = kinds[case % len(kinds)]
-        n = int(rng.integers(1, 200))
-        d = int(rng.integers(1, 6)) * 8 if scalar == "b1" else int(rng.integers(1, 41))
-        m = int(rng.integers(2, 9))
-        ef = int(rng.integers(1, 40))
-        k = int(rng.integers(1, 25))
-        base, q = common.make_collection(n, d, scalar, 16, seed=100 + case, rank=min(4, d))
-        if n > 4:
-            base[n // 2] = base[0]                                  # a duplicate: equal distances
-        keys = rng.permutation(np.arange(10 * n, dtype=np.uint64))[:n]
-        ref, _ = common.build_reference_blob(base, metric, scalar, d, m, expansion_add=int(rng.integers(2, 40)), threads=1, keys=keys)
-        for key in keys[:int(rng.integers(0, max(1, n // 3)))]:
+    for case, c in enumerate(common.small_random_cases()):
+        metric, scalar, n, d, m, ef, k, q = (c[f] for f in ("metric", "scalar", "n", "d", "m", "ef", "k", "q"))
+        ref, _ = common.build_reference_blob(c["base"], metric, scalar, d, m, expansion_add=c["expansion_add"], threads=1,
+                                             keys=c["keys"])
+        for key in c["removed"]:
             ref.remove(int(key))
         blob = ref.save()
         ref.pin_metric(True)
@@ -223,3 +254,92 @@ def test_port_matches_live_reference_on_random_small_cases():
                 for a, b in zip(ref.cluster(q, level), port.cluster(q, level)):
                     assert np.array_equal(a.view(np.uint32) if a.dtype == np.float32 else a,
                                           b.view(np.uint32) if b.dtype == np.float32 else b), what + f" cluster {level}"
+
+
+# ---- the same configurations against tests/golden/reference_cases.npz (make_golden_reference_cases.py) -----------------
+
+def _golden_blob(g, *inputs):
+    assert common.digest(*inputs) == str(g["inputs_sha256"]), "the seeded collection came out different on this host"
+    return common.with_vectors(g["graph"], inputs[0])
+
+
+def _assert_search_and_exact(g, port, q, k, what):
+    want = tuple(g[f"search_{f}"] for f in ("keys", "distances", "counts", "computed", "visited"))
+    common.assert_same_results(want, port.search(q, k, threads=2), what)
+    want = tuple(g[f"exact_{f}"] for f in ("keys", "distances", "counts"))
+    common.assert_same_results(want, port.search(q, k, threads=2, exact=True)[:3], what + " exact")
+
+
+def _assert_cluster(g, port, q, what):
+    for i, level in enumerate(g["cluster_levels"]):
+        got = port.cluster(q, int(level))
+        for field, b in zip(("keys", "distances", "computed", "visited"), got):
+            a = g[f"cluster_{field}"][i]
+            assert np.array_equal(a.view(np.uint32) if a.dtype == np.float32 else a,
+                                  b.view(np.uint32) if b.dtype == np.float32 else b), f"{what} cluster level {level} {field}"
+
+
+@pytest.mark.parametrize("name,metric,scalar,n,d,m,ef,k", common.GOLDEN_SEARCH_CASES, ids=[c[0] for c in common.GOLDEN_SEARCH_CASES])
+def test_port_matches_golden_reference_cases(name, metric, scalar, n, d, m, ef, k):
+    """The configurations of test_port_matches_live_reference (every scalar kind, ef < k, M = 3, 64-bit codes, M = 64):
+    graph and exact search of the port on the reference's graph against what the reference returned."""
+    g = common.golden_case(name)
+    base, q = common.make_collection(n, d, scalar, common.GOLDEN_NQ, iid=(d < 32))
+    port = bindings.PortIndex(_golden_blob(g, base, q), ef)
+    assert (port.size, port.dims, port.connectivity) == (n, d, m)
+    _assert_search_and_exact(g, port, q, k, name)
+
+
+@pytest.mark.parametrize("name,metric,scalar,n,d,m", common.GOLDEN_CLUSTER_CASES, ids=[c[0] for c in common.GOLDEN_CLUSTER_CASES])
+def test_port_cluster_matches_golden_reference_cases(name, metric, scalar, n, d, m):
+    """index_gt::cluster on several graph levels (up to and beyond the top) against what the reference returned."""
+    g = common.golden_case(name)
+    base, q = common.make_collection(n, d, scalar, common.GOLDEN_NQ)
+    port = bindings.PortIndex(_golden_blob(g, base, q), 64)
+    assert port.max_level >= 3 and int(g["cluster_levels"][3]) == port.max_level
+    _assert_cluster(g, port, q, name)
+
+
+def test_exact_search_oracles_agree_golden():
+    """The port's two brute-force paths against the reference's: index search(exact=True) and exact_search_t over the raw
+    rows; for this symmetric metric the reference's two give the same distance bits."""
+    g = common.golden_case("free_l2sq_f32")
+    base, q = common.make_collection(300, 48, "f32", common.GOLDEN_NQ, iid=True)
+    port = bindings.PortIndex(_golden_blob(g, base, q), 64)
+    want = tuple(g[f"exact_{f}"] for f in ("keys", "distances", "counts"))
+    common.assert_same_results(want, port.search(q, 10, threads=2, exact=True)[:3], "port exact vs reference exact")
+    fk, fd = bindings.port_exact_search(base, q, 10, metric="l2sq", scalar="f32", dims=48)
+    assert np.array_equal(fd.view(np.uint32), g["free_distances"].view(np.uint32))
+    assert np.array_equal(fk, g["free_keys"])  # iid floats: no equal distances
+    assert np.array_equal(g["free_distances"].view(np.uint32), g["exact_distances"].view(np.uint32))
+
+
+def test_pinned_metrics_equal_native_golden():
+    """The reference's NATIVE SimSIMD kernels on an AVX-512 host (distances stored in the golden file) against the pinned
+    restatement: bit for bit for every exactly reproducible metric, cosine within the rsqrt approximation (1 ULP)."""
+    g = common.golden_case("native")
+    assert str(g["isa"]) in ("skylake", "ice", "sapphire", "genoa"), str(g["isa"])
+    for metric, scalar, d, x in common.native_metric_rows():
+        assert common.digest(x) == str(g[f"{metric}_{scalar}_sha256"]), (metric, scalar)
+        empty = v2format.Graph(metric, scalar, d, 4, 8, np.zeros((0, x.shape[1] * x.itemsize), np.uint8),
+                               np.zeros(0, np.uint64), np.zeros(0, np.int16), [], 0, 0)
+        port = bindings.PortIndex(v2format.dumps(empty))
+        pinned = np.array([port.distance(x[i], x[i + 1]) for i in range(len(x) - 1)], dtype=np.float32)
+        native = g[f"{metric}_{scalar}"]
+        if metric == "cos":
+            assert ulp_distance(native, pinned).max() <= 1, (metric, scalar)
+        else:
+            assert np.array_equal(native.view(np.uint32), pinned.view(np.uint32)), (metric, scalar)
+
+
+def test_port_matches_golden_random_small_cases():
+    """The first seeded random configurations of test_port_matches_live_reference_on_random_small_cases (n from 1, k > n,
+    ef < k, removed members, duplicate vectors, every scalar kind): graph search, exact search and cluster of the port
+    against what the reference returned."""
+    for case, c in zip(range(common.GOLDEN_SMALL_CASES), common.small_random_cases()):
+        g = common.golden_case(f"small_{case}")
+        what = f"case {case}: {c['metric']}/{c['scalar']} n={c['n']} d={c['d']} M={c['m']} ef={c['ef']} k={c['k']}"
+        port = bindings.PortIndex(_golden_blob(g, c["base"], c["q"]), c["ef"])
+        _assert_search_and_exact(g, port, c["q"], c["k"], what)
+        if "cluster_levels" in g:
+            _assert_cluster(g, port, c["q"], what)

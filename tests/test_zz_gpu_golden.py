@@ -75,10 +75,10 @@ def test_next_rows_match_golden(path):
 ])
 def test_short_vector_kernels_match_reference(metric, scalar, n, d, m, ef, k, nq):
     """The kernels that became the default in round 2 for f16 / bf16 / i8 (search_kernel.cu, dispatch) against the pinned
-    oracle on a reference-built graph: labels, distance bits, counts, both counters."""
+    oracle: labels, distance bits, counts, both counters."""
     from usearch_b200.index import Index
     base, q = common.make_collection(n, d, scalar, nq)
-    ref, blob = common.build_reference_blob(base, metric, scalar, d, m, threads=16)
+    blob = common.build_graph_blob(base, metric, scalar, d, m)
     want = bindings.PortIndex(blob, ef).search(q, k, threads=16)
     index = Index.restore(blob)
     index.expansion_search = ef
